@@ -201,8 +201,42 @@ def driver_config(wl):
     return c
 
 
+class _DevBuf:
+    """a device pointer the driver returned, as an object torch.as_tensor can view without a copy"""
+
+    def __init__(self, ptr, nbytes):
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 2}
+
+
+CU_FIELDS = np.dtype([("type", "u1"), ("depth", "u1"), ("part_size", "u1"), ("tr_depth", "u1"), ("tr_skip", "u1"), ("qp", "u1"),
+                      ("mode", "i1"), ("mode_chroma", "i1"), ("cbf", "<u2"), ("pad", "<u2")])        # kvz_cuda_ctu_cu
+DUMP_ELEMENTS = 3_500_000        # per array: four float32 arrays stay under 64 MB
+
+
+def dump_outputs(directory, wl, kept):
+    """kept: {picture index: (cu, coeff, sao, rec) byte tensors on the device} of the last timed step.  Writes the four result
+    arrays of kvz_cuda_ctu_wait_device over those pictures (in picture order) as float32 .npy files; an array larger than
+    DUMP_ELEMENTS is replaced by a fixed sample of its elements (seed 0, the same for every build)."""
+    os.makedirs(directory, exist_ok=True)
+    w, h = wl["w"], wl["h"]
+    order = sorted(kept)
+    cu = np.stack([kept[i][0].cpu().numpy().view(CU_FIELDS) for i in order])
+    arrays = {
+        "cu": np.stack([cu[f] for f in CU_FIELDS.names if f != "pad"], -1).reshape(len(order), (h + 63) // 64 * 16, -1, len(CU_FIELDS) - 1),
+        "coeff": np.stack([kept[i][1].cpu().numpy().view(np.int16) for i in order]),
+        "sao": np.stack([kept[i][2].cpu().numpy().view(np.int32).reshape(-1, 2, 17) for i in order]),
+        "rec": np.stack([kept[i][3].cpu().numpy() for i in order]),
+    }
+    for name, a in arrays.items():
+        a = a.astype(np.float32)
+        if a.size > DUMP_ELEMENTS:
+            a = a.ravel()[np.sort(np.random.default_rng(0).integers(0, a.size, DUMP_ELEMENTS))]
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def device_leg(args, wl, local, frames_per_step, barrier):
-    """`value`: pictures resident in HBM through the driver alone; returns (seconds for K steps, launches, mean search-kernel ms)"""
+    """`value`: pictures resident in HBM through the driver alone; returns (seconds for K steps, launches, mean search-kernel ms,
+    slots, and with --dump-outputs the results of the last timed step's pictures as device copies)"""
     import torch
     import kvazaar_b200 as kb
     lib = C.CDLL(kb.LIB_PATH)
@@ -242,6 +276,13 @@ def device_leg(args, wl, local, frames_per_step, barrier):
         e0.record()
     lock = threading.Lock()
     n_threads = min(8, slots)
+    # --dump-outputs: the results of the last timed step's pictures are copied on the device (a side stream, synchronised
+    # before the slot is released) and brought to the host after the run
+    last_step = range(n_warm + n_timed - frames_per_step, n_warm + n_timed) if args.dump_outputs else range(0)
+    kept = {}
+    side = torch.cuda.Stream() if args.dump_outputs else None
+    nctu = ((w + 63) // 64) * ((h + 63) // 64)
+    sizes = ((h + 63) // 64 * 16 * ((w + 63) // 64) * 16 * CU_FIELDS.itemsize, nctu * 6144 * 2, nctu * 2 * 68, w * h * 3 // 2)
 
     def drive(share):
         try:
@@ -260,13 +301,20 @@ def device_leg(args, wl, local, frames_per_step, barrier):
                                                        cfg.lambda_, cfg.lambda_sqrt, wl["qp"])
                     if s < 0:
                         raise RuntimeError(f"submit: {lib.kvz_cuda_last_error()}")
-                    pending.append(s)
+                    pending.append((s, i))
                 if not pending:
                     return
-                s = pending.pop(0)
+                s, i = pending.pop(0)
                 if lib.kvz_cuda_ctu_wait_device(enc, s, C.byref(res)) != 0:
                     raise RuntimeError(f"wait: {lib.kvz_cuda_last_error()}")
                 ms = res.search_kernel_ms
+                if i in last_step:
+                    with torch.cuda.stream(side):
+                        copies = tuple(torch.as_tensor(_DevBuf(p, n), device="cuda").clone()
+                                       for p, n in zip((res.cu, res.coeff, res.sao, res.rec), sizes))
+                    side.synchronize()
+                    with lock:
+                        kept[i] = copies
                 lib.kvz_cuda_ctu_release(enc, s)
                 with lock:
                     state["done"] += 1
@@ -295,7 +343,7 @@ def device_leg(args, wl, local, frames_per_step, barrier):
     l0, l1 = state["l0"], state["l1"]
     launches = int(l1 - l0)
     lib.kvz_cuda_ctu_close(enc)
-    return seconds, launches, float(np.mean(kernel_ms)) if kernel_ms else None, slots
+    return seconds, launches, float(np.mean(kernel_ms)) if kernel_ms else None, slots, kept
 
 
 def run_cuda(args, wl):
@@ -343,8 +391,10 @@ def run_cuda(args, wl):
         r = stream_bench(ctu_bin, clip, wl, f"/tmp/kvz_bench_ctu_{rank}.hevc", fps_step, args.steps, args.warmup, cooldown=owf + 1, extra=extra, env=env)
         e2e_seconds = max_over_ranks(r["seconds"])
         # ---- value: the device side alone
-        dev_seconds, launches, kernel_ms, slots = device_leg(args, wl, local, fps_step, barrier)
+        dev_seconds, launches, kernel_ms, slots, kept = device_leg(args, wl, local, fps_step, barrier)
         dev_seconds = max_over_ranks(dev_seconds)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"), wl, kept)
     # N > 1: the two exchanges of SURVEY 8e (tile all-gather of a 4320p 10-bit picture, reference-frame broadcast) timed on
     # this process group -- they are not on the all-intra data path (pictures shard with no collective), this is their
     # hardware measurement; outside the timed regions, every rank takes part
@@ -441,6 +491,9 @@ def main():
     ap.add_argument("--owf", type=int, default=0, help="pictures the encoder keeps in flight (CUDA arm)")
     ap.add_argument("--slots", type=int, default=0, help="pictures in flight of the device-only leg")
     ap.add_argument("--sample-frames", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="CUDA arm: write the results of the last timed step's pictures (CU records, coefficients, SAO parameters, "
+                         "final picture) to DIR/<name>.npy as float32, so that two builds can be compared")
     args = ap.parse_args()
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":

@@ -55,11 +55,9 @@ def build_oracle(bitdepth=8):
 
 
 def build_ref(bitdepth=8):
-    """Build oracle/_ref from /root/reference when it is present (this container);
-    on the GPU box the prebuilt files travel with the snapshot."""
+    """The compiled reference shim that __graft_entry__.build() made under oracle/_ref (when the reference sources were
+    there to build it from), or None; tests never compile the reference themselves."""
     so = os.path.join(REF_DIR, "libkvzref_shim.so" if bitdepth == 8 else "libkvzref_shim_10b.so")
-    if os.path.isdir("/root/reference/src"):
-        subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "ref", "-j8", f"BITDEPTH={bitdepth}"])
     return so if os.path.exists(so) else None
 
 
@@ -393,7 +391,7 @@ class Ref:
     def __init__(self, bitdepth=8):
         so = build_ref(bitdepth)
         if so is None:
-            raise FileNotFoundError("oracle/_ref not built and /root/reference absent")
+            raise FileNotFoundError("oracle/_ref not built (build() builds it when the reference sources are present)")
         self.lib = C.CDLL(so)
         L = self.lib
         L.kvzref_find.restype = C.c_void_p

@@ -245,41 +245,49 @@ def test_reference_frame_pass_10bit_runs(ref10):
     assert api.fp_section(a, sec, "sao_rec").max() > 255 and api.fp_section(a, sec, "checksum").any()
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("dims,qp,signhide,rdoq,trskip", [((136, 72), 30, 0, 0, 0), ((200, 136), 27, 1, 1, 0), ((320, 192), 34, 1, 1, 1)])
-def test_cuda10_frame_pass_matches_reference(cuda_lib, ref10, dims, qp, signhide, rdoq, trskip):
-    """The whole frame-level pass on 10-bit samples (config-5 bit depth): blob identical to the pass through the 10-bit
-    reference build's strategy functions."""
+PARITY10_CASES = [((136, 72), 30, 0, 0, 0), ((200, 136), 27, 1, 1, 0), ((320, 192), 34, 1, 1, 1)]
+# the configs[4] shape at its full size: (dims, qp, signhide, rdoq, trskip, frame index)
+FULL_SIZE10_CASE = ((7680, 4320), 22, 0, 1, 0, 3)
+
+
+@pytest.mark.parametrize("dims,qp,signhide,rdoq,trskip", PARITY10_CASES)
+def test_reference_frame_pass_10bit_matches_golden(ref10, dims, qp, signhide, rdoq, trskip):
+    """the digests the GPU tests compare with are those of the 10-bit reference build's own pass"""
+    from _golden import assert_matches_reference, fp_case
     from _oracle import ref_frame_pass
+    from kvazaar_b200 import api
+    W, H = dims
+    lay = api.fp_layout_for(W, H, qp, signhide, 10)
+    want = ref_frame_pass(ref10, synth_frame10(W, H, W + qp), W, H, qp, lay, nthreads=4, signhide=signhide, rdoq=rdoq, trskip=trskip)
+    assert_matches_reference(want, api.fp_sections(lay, W, H, 10), fp_case(W, H, qp, signhide, rdoq, trskip, 10))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dims,qp,signhide,rdoq,trskip", PARITY10_CASES)
+def test_cuda10_frame_pass_matches_reference(cuda_lib, dims, qp, signhide, rdoq, trskip):
+    """The whole frame-level pass on 10-bit samples (config-5 bit depth): blob identical to the pass through the 10-bit
+    reference build's strategy functions (its digests, tests/_golden.py)."""
+    from _golden import assert_matches_reference, fp_case
     kb = cuda_lib
     W, H = dims
     src = synth_frame10(W, H, W + qp)
     fp = kb.FramePass(W, H, qp, signhide, rdoq, 0.0, trskip, 10)
     fp.run_dev(kb.to_dev(src))
     got = fp.result_host()
-    want = ref_frame_pass(ref10, src, W, H, qp, fp.layout, nthreads=4, signhide=signhide, rdoq=rdoq, trskip=trskip)
-    sec = kb.fp_sections(fp.layout, W, H, 10)
-    for name in sec:
-        a, b = kb.fp_section(got, sec, name), kb.fp_section(want, sec, name)
-        assert np.array_equal(a, b), (name, int(np.argmax(a != b)), a[a != b][:4], b[a != b][:4])
+    assert_matches_reference(got, kb.fp_sections(fp.layout, W, H, 10), fp_case(W, H, qp, signhide, rdoq, trskip, 10))
     fp.close()
 
 
 @pytest.mark.gpu
-def test_cuda10_frame_pass_full_size_4320p(cuda_lib, ref10):
+def test_cuda10_frame_pass_full_size_4320p(cuda_lib):
     """The configs[4] shape at its full size (7680x4320 10-bit, QP22, RDOQ + deblocking + SAO): one frame, every section of
-    the result blob equals the pass through the 10-bit reference build's strategy functions."""
-    import os
-    from _oracle import ref_frame_pass
+    the result blob equals the pass through the 10-bit reference build's strategy functions (its digests, tests/_golden.py)."""
+    from _golden import assert_matches_reference, fp_case
     kb = cuda_lib
-    W, H, qp = 7680, 4320, 22
-    src = synth_frame10(W, H, 3)
-    fp = kb.FramePass(W, H, qp, 0, 1, 0.0, 0, 10)
+    (W, H), qp, signhide, rdoq, trskip, idx = FULL_SIZE10_CASE
+    src = synth_frame10(W, H, idx)
+    fp = kb.FramePass(W, H, qp, signhide, rdoq, 0.0, trskip, 10)
     fp.run_dev(kb.to_dev(src))
     got = fp.result_host()
-    want = ref_frame_pass(ref10, src, W, H, qp, fp.layout, nthreads=min(64, os.cpu_count() or 8), signhide=0, rdoq=1, trskip=0)
-    sec = kb.fp_sections(fp.layout, W, H, 10)
-    for name in sec:
-        a, b = kb.fp_section(got, sec, name), kb.fp_section(want, sec, name)
-        assert np.array_equal(a, b), (name, int(np.argmax(a != b)))
+    assert_matches_reference(got, kb.fp_sections(fp.layout, W, H, 10), fp_case(W, H, qp, signhide, rdoq, trskip, 10))
     fp.close()

@@ -132,9 +132,8 @@ def test_ctu_driver_pictures_shard_over_ranks_gloo_world2(tmp_path):
         if not os.path.exists(os.path.join(root, "oracle", "_ref", f)):
             import pytest
             pytest.skip("oracle/_ref stream bench hosts missing")
-    if not os.path.exists(os.path.join(root, "tests", "hostsim", "libkvzctu_hostsim.so")):
-        import subprocess
-        subprocess.check_call(["sh", os.path.join(root, "tools", "build_hostsim.sh")])
+    from test_ctu_driver import _hostsim
+    _hostsim()                                                  # builds the host library if it is missing
     sys.path.insert(0, os.path.join(root, "tools"))
     from synth_yuv import synth_frame
     clip = str(tmp_path / "c.yuv")

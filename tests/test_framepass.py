@@ -83,42 +83,63 @@ def test_reference_frame_pass_is_self_consistent(ref, orc):
     assert np.array_equal(blob, blob1)
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("dims,qp,signhide,rdoq", [((136, 72), 27, 0, 0), ((200, 136), 27, 0, 0), ((320, 192), 27, 0, 0),
-                                                    ((200, 136), 22, 1, 0), ((136, 72), 37, 1, 0), ((320, 192), 17, 1, 0),
-                                                    ((200, 136), 27, 0, 1), ((320, 192), 22, 1, 1), ((136, 72), 32, 0, 1),
-                                                    ((320, 192), 22, 1, 3), ((200, 136), 27, 0, 2), ((136, 72), 17, 1, 3)])
-def test_cuda_frame_pass_matches_reference(cuda_lib, ref, dims, qp, signhide, rdoq):
-    """Byte-identical result blob: CUDA frame pass vs the reference's own strategy functions (medium-like:
-    signhide off; veryslow-like: QP 22 with sign-bit hiding; rdoq = 1: kvz_rdoq instead of kvz_quant, as medium and
-    veryslow configure it)."""
-    import torch
-    from _oracle import ref_frame_pass
-    kb = cuda_lib
-    W, H = dims
-    trskip, rdoq = rdoq >> 1, rdoq & 1                     # bit 1 of the parameter: also try transform skip on 4x4 luma (veryslow)
+PARITY_CASES = [((136, 72), 27, 0, 0), ((200, 136), 27, 0, 0), ((320, 192), 27, 0, 0),
+                ((200, 136), 22, 1, 0), ((136, 72), 37, 1, 0), ((320, 192), 17, 1, 0),
+                ((200, 136), 27, 0, 1), ((320, 192), 22, 1, 1), ((136, 72), 32, 0, 1),
+                ((320, 192), 22, 1, 3), ((200, 136), 27, 0, 2), ((136, 72), 17, 1, 3)]
+# the BASELINE configs[1] and configs[2] shapes at their full sizes: (dims, qp, signhide, rdoq, trskip, frame_idx)
+FULL_SIZE_CASES = {"1080p_medium": ((1920, 1080), 27, 0, 1, 0, 5), "2160p_veryslow": ((3840, 2160), 22, 1, 1, 1, 7)}
+
+
+def parity_frame(W, H, qp, trskip):
+    """the source of a PARITY_CASES case"""
     src = synth_frame(W, H, frame_idx=W + qp)
     if trskip:                                              # text-like content in a corner so that transform skip wins somewhere
         y = src[:W * H].reshape(H, W)
         y[:64, :64] = np.where((np.add.outer(np.arange(64), np.arange(64)) // 3) % 2, 40, 220).astype(np.uint8)
+    return src
+
+
+@pytest.mark.parametrize("dims,qp,signhide,rdoq", PARITY_CASES)
+def test_reference_frame_pass_matches_golden(ref, dims, qp, signhide, rdoq):
+    """the digests the GPU tests compare with are those of the reference's own pass"""
+    import kvazaar_b200 as kb
+    from _golden import assert_matches_reference, fp_case
+    from _oracle import ref_frame_pass
+    W, H = dims
+    trskip, rdoq = rdoq >> 1, rdoq & 1
+    lay = kb.fp_layout_for(W, H, qp, signhide)
+    want = ref_frame_pass(ref, parity_frame(W, H, qp, trskip), W, H, qp, lay, nthreads=4, signhide=signhide, rdoq=rdoq, trskip=trskip)
+    assert_matches_reference(want, kb.fp_sections(lay, W, H), fp_case(W, H, qp, signhide, rdoq, trskip))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dims,qp,signhide,rdoq", PARITY_CASES)
+def test_cuda_frame_pass_matches_reference(cuda_lib, dims, qp, signhide, rdoq):
+    """Byte-identical result blob: CUDA frame pass vs the reference's own strategy functions (medium-like:
+    signhide off; veryslow-like: QP 22 with sign-bit hiding; rdoq = 1: kvz_rdoq instead of kvz_quant, as medium and
+    veryslow configure it), through the digests of the reference's blob (tests/_golden.py)."""
+    import torch
+    from _golden import assert_matches_reference, fp_case
+    kb = cuda_lib
+    W, H = dims
+    trskip, rdoq = rdoq >> 1, rdoq & 1                     # bit 1 of the parameter: also try transform skip on 4x4 luma (veryslow)
+    case = fp_case(W, H, qp, signhide, rdoq, trskip)
+    src = parity_frame(W, H, qp, trskip)
     fp = kb.FramePass(W, H, qp, signhide, rdoq, 0.0, trskip)
     fp.run_dev(kb.to_dev(src))
     got = fp.result_host()
-    want = ref_frame_pass(ref, src, W, H, qp, fp.layout, nthreads=4, signhide=signhide, rdoq=rdoq, trskip=trskip)
-    if trskip:
-        flags = kb.fp_section(want, kb.fp_sections(fp.layout, W, H), "trskip_y")
-        assert 0 < int(flags.sum()) < flags.size, "transform skip never (or always) chosen: the case does not exercise the choice"
     sec = kb.fp_sections(fp.layout, W, H)
-    for name in sec:
-        a, b = kb.fp_section(got, sec, name), kb.fp_section(want, sec, name)
-        assert np.array_equal(a, b), (name, int(np.argmax(a != b)), a[a != b][:4], b[a != b][:4])
+    assert_matches_reference(got, sec, case)
+    if trskip:
+        flags = kb.fp_section(got, sec, "trskip_y")
+        assert 0 < int(flags.sum()) < flags.size, "transform skip never (or always) chosen: the case does not exercise the choice"
     # host-buffer entry point gives the same blob
     src_pin = torch.from_numpy(src.copy()).pin_memory()
     res_pin = torch.empty(fp.host_bytes, dtype=torch.uint8).pin_memory()
     fp.run_host(src_pin, res_pin)
     torch.cuda.synchronize()
-    for name in sec:
-        assert np.array_equal(kb.fp_section(res_pin.numpy(), sec, name), kb.fp_section(want, sec, name)), name
+    assert_matches_reference(res_pin.numpy(), sec, case)
     # compact result (bitmap + non-zero coefficient chunks) expands to the same blob
     L = fp.layout
     assert int(L.coeff_begin) + 32 * int(L.n_chunks) == fp.host_bytes
@@ -134,25 +155,21 @@ def test_cuda_frame_pass_matches_reference(cuda_lib, ref, dims, qp, signhide, rd
 
 
 @pytest.mark.gpu
-def test_cuda_frame_pass_full_size_1080p_medium(cuda_lib, ref):
+def test_cuda_frame_pass_full_size_1080p_medium(cuda_lib):
     """BASELINE configs[1] at its full size (1920x1080, QP27, RDOQ + deblocking + SAO): every section of the result blob
-    equals the pass through the reference's strategy functions; the compact result expands to the same bytes."""
-    import os
+    equals the pass through the reference's strategy functions (its digests, tests/_golden.py); the compact result expands
+    to the same bytes."""
     import torch
-    from _oracle import ref_frame_pass
+    from _golden import assert_matches_reference, fp_case
     kb = cuda_lib
-    W, H, qp = 1920, 1080, 27
-    src = synth_frame(W, H, frame_idx=5)
-    fp = kb.FramePass(W, H, qp, 0, 1)
+    (W, H), qp, signhide, rdoq, trskip, idx = FULL_SIZE_CASES["1080p_medium"]
+    src = synth_frame(W, H, frame_idx=idx)
+    fp = kb.FramePass(W, H, qp, signhide, rdoq, 0.0, trskip)
     src_pin = torch.from_numpy(src.copy()).pin_memory()
     res_pin = torch.empty(fp.host_bytes, dtype=torch.uint8).pin_memory()
     fp.run_host(src_pin, res_pin)
     torch.cuda.synchronize()
-    want = ref_frame_pass(ref, src, W, H, qp, fp.layout, nthreads=min(64, os.cpu_count() or 8), signhide=0, rdoq=1)
-    sec = kb.fp_sections(fp.layout, W, H)
-    for name in sec:
-        a, b = kb.fp_section(res_pin.numpy(), sec, name), kb.fp_section(want, sec, name)
-        assert np.array_equal(a, b), (name, int(np.argmax(a != b)))
+    assert_matches_reference(res_pin.numpy(), kb.fp_sections(fp.layout, W, H), fp_case(W, H, qp, signhide, rdoq, trskip))
     L = fp.layout
     small = torch.zeros(int(L.coeff_begin), dtype=torch.uint8).pin_memory()
     compact = torch.zeros(int(L.compact_header_bytes) + 32 * (int(L.n_chunks) // 8), dtype=torch.uint8).pin_memory()
@@ -163,23 +180,19 @@ def test_cuda_frame_pass_full_size_1080p_medium(cuda_lib, ref):
 
 
 @pytest.mark.gpu
-def test_cuda_frame_pass_full_size_2160p_veryslow_shape(cuda_lib, ref):
+def test_cuda_frame_pass_full_size_2160p_veryslow_shape(cuda_lib):
     """The configs[2] shape at its full size (3840x2160, QP22, RDOQ + sign hiding + transform-skip choice + deblocking +
-    SAO): one frame, every section of the result blob equals the pass through the reference's strategy functions."""
-    import os
+    SAO): one frame, every section of the result blob equals the pass through the reference's strategy functions (its
+    digests, tests/_golden.py)."""
     import torch
-    from _oracle import ref_frame_pass
+    from _golden import assert_matches_reference, fp_case
     kb = cuda_lib
-    W, H, qp = 3840, 2160, 22
-    src = synth_frame(W, H, frame_idx=7)
-    fp = kb.FramePass(W, H, qp, 1, 1, 0.0, 1)
+    (W, H), qp, signhide, rdoq, trskip, idx = FULL_SIZE_CASES["2160p_veryslow"]
+    src = synth_frame(W, H, frame_idx=idx)
+    fp = kb.FramePass(W, H, qp, signhide, rdoq, 0.0, trskip)
     src_pin = torch.from_numpy(src.copy()).pin_memory()
     res_pin = torch.empty(fp.host_bytes, dtype=torch.uint8).pin_memory()
     fp.run_host(src_pin, res_pin)
     torch.cuda.synchronize()
-    want = ref_frame_pass(ref, src, W, H, qp, fp.layout, nthreads=min(64, os.cpu_count() or 8), signhide=1, rdoq=1, trskip=1)
-    sec = kb.fp_sections(fp.layout, W, H)
-    for name in sec:
-        a, b = kb.fp_section(res_pin.numpy(), sec, name), kb.fp_section(want, sec, name)
-        assert np.array_equal(a, b), (name, int(np.argmax(a != b)))
+    assert_matches_reference(res_pin.numpy(), kb.fp_sections(fp.layout, W, H), fp_case(W, H, qp, signhide, rdoq, trskip))
     fp.close()

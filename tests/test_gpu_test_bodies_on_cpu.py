@@ -42,12 +42,22 @@ def test_fractional_test_bodies(kb, ref, ref10):
 
 
 def test_bench_me_bookkeeping(kb, monkeypatch):
-    """tools/bench_me.py's measure() with the stand-in: every stage reports `identical`"""
+    """tools/bench_me.py's measure() with the stand-in: every stage reports `identical` against the reference's outputs for
+    the same run, committed as tests/golden/bench_me_416x240.npz (tools/make_golden_me.py)"""
+    import os
     import time
+    import numpy as np
     import kvazaar_b200
     import bench_me
+    import me_cases
     for name in ("init", "to_dev", "me_search_batch", "me_frac_search_batch", "me_candidates_batch", "me_merge_cost_batch"):
         monkeypatch.setattr(kvazaar_b200, name, getattr(kb, name), raising=False)
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "bench_me_416x240.npz"))
+    monkeypatch.setattr(me_cases, "RefShim", lambda bitdepth=8: None)
+    monkeypatch.setattr(me_cases, "run_reference", lambda *a: g["integer"].view(me_cases.RESULT))
+    monkeypatch.setattr(me_cases, "run_frac_reference", lambda *a: g["fractional"].view(me_cases.RESULT))
+    monkeypatch.setattr(me_cases, "run_cand_reference", lambda *a: g["candidates"].view(me_cases.CAND_OUT))
+    monkeypatch.setattr(me_cases, "run_merge_reference", lambda *a: (g["merge"].view(me_cases.MERGE_COST), tuple(g["merge_bits"])))
 
     def timed(fn, iters):
         t = time.perf_counter()

@@ -43,27 +43,39 @@ def test_reference_inter_pass_finds_the_motion(ref):
     assert np.array_equal(blob, blob1)
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("dims,qp,rng", [((128, 96), 27, 8), ((208, 136), 32, 5), ((320, 192), 22, 8)])
-def test_cuda_inter_pass_matches_reference(cuda_lib, ref, dims, qp, rng):
-    """Byte-identical result blob: CUDA inter pass vs the reference's own strategy functions."""
-    import torch
+PARITY_CASES = [((128, 96), 27, 8), ((208, 136), 32, 5), ((320, 192), 22, 8)]
+
+
+@pytest.mark.parametrize("dims,qp,rng", PARITY_CASES)
+def test_reference_inter_pass_matches_golden(ref, dims, qp, rng):
+    """the digests the GPU tests compare with are those of the reference's own pass"""
+    import kvazaar_b200 as kb
+    from _golden import assert_matches_reference, ip_case
     from _oracle import ref_inter_pass
+    W, H = dims
+    cur, rf = moving_pair(W, H, seed=W)
+    lay = kb.ip_layout_for(W, H, qp, rng)
+    want = ref_inter_pass(ref, cur, rf, W, H, qp, rng, lay, nthreads=4)
+    assert_matches_reference(want, kb.ip_sections(lay, W, H), ip_case(W, H, qp, rng))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dims,qp,rng", PARITY_CASES)
+def test_cuda_inter_pass_matches_reference(cuda_lib, dims, qp, rng):
+    """Byte-identical result blob: CUDA inter pass vs the reference's own strategy functions (its digests, tests/_golden.py)."""
+    import torch
+    from _golden import assert_matches_reference, ip_case
     kb = cuda_lib
     W, H = dims
     cur, rf = moving_pair(W, H, seed=W)
     ip = kb.InterPass(W, H, qp, rng)
     ip.run_dev(kb.to_dev(cur), kb.to_dev(rf))
     got = ip.result_host()
-    want = ref_inter_pass(ref, cur, rf, W, H, qp, rng, ip.layout, nthreads=4)
     sec = kb.ip_sections(ip.layout, W, H)
-    for name in sec:
-        a, b = kb.fp_section(got, sec, name), kb.fp_section(want, sec, name)
-        assert np.array_equal(a, b), (name, int(np.argmax(a != b)), a[a != b][:6], b[a != b][:6])
+    assert_matches_reference(got, sec, ip_case(W, H, qp, rng))
     cur_pin, ref_pin = torch.from_numpy(cur.copy()).pin_memory(), torch.from_numpy(rf.copy()).pin_memory()
     res_pin = torch.empty(ip.host_bytes, dtype=torch.uint8).pin_memory()
     ip.run_host(cur_pin, ref_pin, res_pin)
     torch.cuda.synchronize()
-    for name in sec:
-        assert np.array_equal(kb.fp_section(res_pin.numpy(), sec, name), kb.fp_section(want, sec, name)), name
+    assert_matches_reference(res_pin.numpy(), sec, ip_case(W, H, qp, rng))
     ip.close()

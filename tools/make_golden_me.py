@@ -54,3 +54,29 @@ for name in sorted(MC_CASES):
     out["mc/" + name] = np.frombuffer(b"".join(hashlib.sha256(a.tobytes()).digest() for a in (oy, ou, ov)), np.uint8).copy()      # sha256 of Y, U, V
     print("mc", name, len(pus), "PUs")
 np.savez_compressed(os.path.join(ROOT, "tests", "golden", "me_search.npz"), **out)
+
+# tests/golden/bench_me_416x240.npz: what the reference returns in tools/bench_me.py's measure("416x240", 16, "hexbs", 8, 1, 4),
+# the run tests/test_gpu_test_bodies_on_cpu.py checks with the host build of the device code standing in for the device
+import bench_me  # noqa: E402
+import kvazaar_b200  # noqa: E402
+import me_cases  # noqa: E402
+from _fake_kb import FakeKB  # noqa: E402
+
+fake = FakeKB()
+for n in ("init", "to_dev", "me_search_batch", "me_frac_search_batch", "me_candidates_batch", "me_merge_cost_batch"):
+    setattr(kvazaar_b200, n, getattr(fake, n))
+bench_me.timed = lambda fn, iters: (fn(), 1.0)[1]
+recorded = {}
+for key, name in (("integer", "run_reference"), ("fractional", "run_frac_reference"), ("candidates", "run_cand_reference"), ("merge", "run_merge_reference")):
+    def recording(*a, _key=key, _fn=getattr(me_cases, name)):
+        recorded[_key] = _fn(*a)
+        return recorded[_key]
+    setattr(me_cases, name, recording)
+line = bench_me.measure("416x240", 16, "hexbs", 8, 1, 4, True)
+assert all(line[k]["identical"] for k in ("integer", "fractional", "candidates", "merge_analysis")), line
+merge, merge_bits = recorded.pop("merge")
+bench = {k: np.frombuffer(v.tobytes(), np.uint8).copy() for k, v in recorded.items()}
+bench["merge"] = np.frombuffer(merge.tobytes(), np.uint8).copy()
+bench["merge_bits"] = np.array(merge_bits, np.float64)
+np.savez_compressed(os.path.join(ROOT, "tests", "golden", "bench_me_416x240.npz"), **bench)
+print("bench_me 416x240:", {k: v.size for k, v in bench.items()})
